@@ -2,6 +2,7 @@
 """bench.py -- NNConv edge-applications/s on synthetic Darcy-2D radius graphs (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload darcy241|darcy85]
+                    [--dump-outputs DIR]
 
 One "step" = one KernelNN conv stack (T applications of the shared NNConv, graph-neural-operator/
 UAI1_full_resolution.py:29-30) over ONE graph sample per GPU: the x-independent edge features are
@@ -10,8 +11,14 @@ value = (ranks x E x T x K) / max-over-ranks device time  [edge-applications/s],
 e2e   = same through the public module call KernelNN.forward with pinned-host inputs copied H2D and the
         result read back D2H inside the timed region, every step.
 Weak scaling: every rank owns its own graph sample(s); no data-path collective (batch sharding).
+--steps K sets the timed steps of value and e2e (the metric); the secondary lines keep fixed step counts: train
+2..3 steps (K clamped), fp32_grade 3, configs 3-50 repetitions, gpu_reference_port 1, cpu_baseline 2, strip 2..5.
 --impl reference: the CPU oracle port (oracle/nnconv_oracle.py, torch CPU, all host threads) on a bounded
 sample of the same workload (rank 0 only).
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step of each timed path returned,
+DIR/conv_stack.npy (resident path: node features after the T applications, [N, width]) and DIR/model_out.npy
+(e2e path: KernelNN.forward, [N, 1]), float32.  Inputs and weights are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -105,7 +112,7 @@ REF_SAMPLE_SOURCES = 192     # fixed, so that reference-arm numbers are comparab
 
 def cpu_reference_rate(cfg, steps=1, warmup=0, n_src=REF_SAMPLE_SOURCES):
     """The reference's CPU path on a bounded, FIXED sample: out-edges of the first n_src source nodes of the
-    workload graph, T applications of one NNConv.  Runs the reference's OWN files (baseline/_ref, vendored
+    workload graph, T applications of one NNConv.  Runs the reference's OWN files (oracle/_ref, vendored
     unmodified by oracle/vendor_ref.py; kind 'reference') over oracle/pyg_stub, exactly as the reference runs them
     (one shot over all edges of the sample, torch CPU fp32); falls back to the oracle port (kind 'port') only when
     the vendored copy is absent.  Returns (edge_apps_per_s, cores, kind, sample_description, ms_per_step)."""
@@ -243,6 +250,18 @@ def _time_ms(fn, reps, warm=3):
     b.record()
     torch.cuda.synchronize()
     return a.elapsed_time(b) / reps
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Write {name: tensor} as path/<name>.npy in float32 (darcy241: 15 MB in all)."""
+    arrays = {name: t.detach().float().cpu().numpy() for name, t in arrays.items()}
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES, 'outputs larger than DUMP_MAX_BYTES'
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 def other_configs(dev, precision):
@@ -461,7 +480,8 @@ def run_strip_children(args, rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=5)
+    ap.add_argument('--steps', type=int, default=5,
+                    help='timed steps of the metric and e2e lines (secondary lines: fixed counts, see the docstring)')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--workload', default=os.environ.get('NNCONV_BENCH_WORKLOAD', 'darcy241'), choices=sorted(WORKLOADS))
@@ -472,7 +492,12 @@ def main():
     ap.add_argument('--no-other-configs', action='store_true', help='skip BASELINE configs 2, 4, 5')
     ap.add_argument('--no-strip', action='store_true', help='skip the single-mesh strip-partition measurement (N > 1)')
     ap.add_argument('--strip-only', action='store_true', help=argparse.SUPPRESS)
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the outputs of the b200 arm')
     if args.strip_only:
         return strip_child_main(args)
     cfg = WORKLOADS[args.workload]
@@ -570,7 +595,9 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(fn, steps, warmup, pre=None):
+    last = {}                 # what the last timed step of each path returned (--dump-outputs)
+
+    def timed(fn, steps, warmup, pre=None, keep=False):
         for i in range(warmup):
             fn(i)
         barrier()
@@ -579,7 +606,10 @@ def main():
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
         for i in range(steps):
-            fn(warmup + i)
+            out = fn(warmup + i)
+            if keep:
+                last[fn] = out
+            del out
         b.record()
         barrier()
         ms = torch.tensor([a.elapsed_time(b)], device=dev)
@@ -591,8 +621,10 @@ def main():
     launches0 = nn_conv.stats['launches']
     if rank == 0:
         sampler.start()
-    ms_total = timed(step_resident, args.steps, max(args.warmup, 3))
+    ms_total = timed(step_resident, args.steps, max(args.warmup, 3), keep=bool(args.dump_outputs))
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dumped = {'conv_stack': last.pop(step_resident).cpu()}
     launches = nn_conv.stats['launches'] - launches0
     launches_timed = int(round(launches * args.steps / float(args.steps + max(args.warmup, 3))))
     value = world * E * T * args.steps / (ms_total * 1e-3)
@@ -601,7 +633,12 @@ def main():
         copy_stream.synchronize()
         e2e_state['prefetched'] = -1
 
-    ms_e2e = timed(step_e2e, args.steps, 1, pre=e2e_reset)
+    ms_e2e = timed(step_e2e, args.steps, 1, pre=e2e_reset, keep=bool(args.dump_outputs))
+    if args.dump_outputs:
+        dumped['model_out'] = last.pop(step_e2e).clone()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, dumped)
+        del dumped
     e2e_value = world * E * T * args.steps / (ms_e2e * 1e-3)
     h2d = host_x[0].numel() * 4 + host_ea[0].numel() * 4
     d2h = host_out.numel() * 4

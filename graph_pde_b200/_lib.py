@@ -5,6 +5,7 @@ importing / calling raises.  `build()` compiles the library in-tree with nvcc (s
 """
 import ctypes
 import os
+import shutil
 import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -44,6 +45,8 @@ class NNConvLibraryError(RuntimeError):
 def build(verbose=False):
     """Compile libnnconv_b200.so for sm_100a (nvcc cross-compiles without a GPU)."""
     cmd = ['make', '-C', CSRC, '-j', str(min(8, os.cpu_count() or 1))]
+    if shutil.which('nvcc') is None:      # an account whose PATH lacks the CUDA toolkit's bin directory
+        cmd.append('NVCC=' + os.path.join(os.environ.get('CUDA_HOME', '/usr/local/cuda'), 'bin', 'nvcc'))
     res = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
     if verbose or res.returncode != 0:
         print(res.stdout)

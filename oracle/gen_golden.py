@@ -1,16 +1,18 @@
-"""Generate tests/golden/*.npz by running the REFERENCE's own files, unmodified, in the build container.
+"""Generate tests/golden/*.npz by running the REFERENCE's own files, unmodified.
 
-TEST INFRASTRUCTURE.  Run here only (needs /root/reference, which does not exist on the GPU box):
+TEST INFRASTRUCTURE.  Needs a checkout of the reference (the tests only read the .npz files it writes):
 
-    python oracle/gen_golden.py
+    [GRAPH_PDE_REFERENCE=<reference checkout>] python oracle/gen_golden.py [g1 g2 ... g7]
 
-What runs: /root/reference/graph-neural-operator/{nn_conv.py,utilities.py},
-/root/reference/multipole-graph-neural-operator/utilities.py and the model classes KernelNN /
+(no names: all seven; the checkout defaults to /root/reference).  What runs:
+graph-neural-operator/{nn_conv.py,utilities.py},
+multipole-graph-neural-operator/utilities.py and the model classes KernelNN /
 KernelInduced / MKGN / MGKN extracted (by `ast`, not copied) from the reference scripts, over
 oracle/pyg_stub (the restated third-party boundary, see its docstring).  The outputs are the golden
-vectors that pin oracle/nnconv_oracle.py and, through it, the CUDA path.
+vectors that pin oracle/nnconv_oracle.py and, through it, the CUDA path.  Every file stays under 1 MB.
 """
 import ast
+import hashlib
 import os
 import sys
 import warnings
@@ -20,10 +22,11 @@ import torch
 
 warnings.filterwarnings('ignore')
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = '/root/reference'
+REF = os.environ.get('GRAPH_PDE_REFERENCE') or '/root/reference'      # the reference checkout
 GNO = os.path.join(REF, 'graph-neural-operator')
 MGNO = os.path.join(REF, 'multipole-graph-neural-operator')
 OUT = os.path.join(HERE, '..', 'tests', 'golden')
+WANT = set(a[:2] for a in sys.argv[1:]) or None    # e.g. g3 g4
 
 
 def _import_reference():
@@ -50,7 +53,13 @@ def _np_state(module):
     return {k: v.detach().numpy().copy() for k, v in module.state_dict().items()}
 
 
+def _save(name, **rec):
+    if WANT is None or name[:2] in WANT:
+        np.savez_compressed(os.path.join(OUT, name), **rec)
+
+
 def main():
+    assert os.path.isdir(GNO) and os.path.isdir(MGNO), 'no reference checkout at %s (set GRAPH_PDE_REFERENCE)' % REF
     os.makedirs(OUT, exist_ok=True)
     nn_conv, U, MU = _import_reference()
     import torch.nn.functional as F
@@ -90,7 +99,7 @@ def main():
     rec['oned/x'] = x1.numpy()
     rec['oned/edge_attr'] = ea1.numpy()
     rec['oned/out'] = conv(x1, ei, ea1).detach().numpy()
-    np.savez_compressed(os.path.join(OUT, 'g1_tiny_multigraph.npz'), **rec)
+    _save('g1_tiny_multigraph.npz', **rec)
 
     # ---------------- G2: BASELINE config 1 (16x16, r=.25, w=32, kw=1024, T=4), seeded weights ----
     torch.manual_seed(0)
@@ -120,7 +129,7 @@ def main():
         rec['abs/%s' % k] = np.float64(np.abs(v.astype(np.float64)).sum())
         if v.size <= 8192:
             rec['w/%s' % k] = v
-    np.savez_compressed(os.path.join(OUT, 'g2_cfg1_ball16.npz'), **rec)
+    _save('g2_cfg1_ball16.npz', **rec)
 
     # ---------------- G3: shipped checkpoint weights (the reference's only fixture) ---------------
     import __main__
@@ -130,6 +139,15 @@ def main():
     __main__.KernelNN = KernelNNCkpt
     ck = torch.load(os.path.join(GNO, 'model', 'grain_new_r64_s64testm100'), map_location='cpu',
                     weights_only=False)
+    # the trained 4096 x 128 output layer of the edge network alone is 2 MB: keep the first 32 of the 128 units of
+    # the second hidden layer (edge network 6 -> 64 -> 32 -> 4096, still width 64), so that the file stays < 1 MB
+    k3 = 32
+    lay = ck.conv1.nn.layers
+    with torch.no_grad():
+        lay[2].weight = torch.nn.Parameter(lay[2].weight[:k3].clone())
+        lay[2].bias = torch.nn.Parameter(lay[2].bias[:k3].clone())
+        lay[4].weight = torch.nn.Parameter(lay[4].weight[:, :k3].clone())
+    lay[2].out_features = lay[4].in_features = k3
     st = {k: v.detach().clone() for k, v in ck.state_dict().items()}
     torch.manual_seed(0)
     np.random.seed(0)
@@ -149,7 +167,7 @@ def main():
                x0=xs[0].numpy(), x_after=np.stack([t.numpy() for t in xs[1:]]))
     for k, v in st.items():
         rec['w/%s' % k] = v.numpy()
-    np.savez_compressed(os.path.join(OUT, 'g3_checkpoint_grain_new.npz'), **rec)
+    _save('g3_checkpoint_grain_new.npz', **rec)
 
     # ---------------- G4: MGKN V-cycle (both script variants) on a small multi-level graph ---------
     torch.manual_seed(0)
@@ -173,13 +191,20 @@ def main():
                edge_index_up=ei_up.numpy().astype(np.int32), range_mid=r_mid.numpy(), range_down=r_down.numpy(),
                range_up=r_up.numpy(), edge_attr_mid=ea_mid.numpy(), edge_attr_down=ea_down.numpy(),
                edge_attr_up=ea_up.numpy(), width=32, ker_width=64, depth=2)
+
+    def seeded_state(variant, seed, model):
+        # the untrained parameters are a seeded draw (1.7 MB): stored as seed, shapes and sha256 of their bytes,
+        # the tests re-draw them with the project's constructors (same init stream) and check the hashes
+        rec[variant + '/seed'] = seed
+        for k, v in _np_state(model).items():
+            rec['%s/shape/%s' % (variant, k)] = np.array(v.shape)
+            rec['%s/sha256/%s' % (variant, k)] = np.array(hashlib.sha256(np.ascontiguousarray(v).tobytes()).hexdigest())
     KI = _class_from_script(os.path.join(MGNO, 'neurips1_MGKN.py'), 'KernelInduced', dict(ns_mgno))
     torch.manual_seed(1)
     model = KI(width=32, ker_width=64, depth=2, ker_in=6, points=m, level=level, in_width=6, out_width=1)
     with torch.no_grad():
         rec['neurips1/out'] = model(data).numpy()
-    for k, v in _np_state(model).items():
-        rec['neurips1/w/%s' % k] = v
+    seeded_state('neurips1', 1, model)
     MK = _class_from_script(os.path.join(MGNO, 'MGKN_general_darcy2d.py'), 'MKGN', dict(ns_mgno))
     torch.manual_seed(2)
     import io
@@ -188,9 +213,8 @@ def main():
         model = MK(width=32, ker_width=64, depth=2, ker_in=6, points=m, level=level, in_width=6, out_width=1)
     with torch.no_grad():
         rec['general/out'] = model(data).numpy()
-    for k, v in _np_state(model).items():
-        rec['general/w/%s' % k] = v
-    np.savez_compressed(os.path.join(OUT, 'g4_mgkn_vcycle.npz'), **rec)
+    seeded_state('general', 2, model)
+    _save('g4_mgkn_vcycle.npz', **rec)
 
     # ---------------- G5: orthogonal MGKN, Burgers 1-D multipole graph -----------------------------
     torch.Tensor.cuda = lambda self, *a, **k: self      # reference calls .cuda() (MGNO/utilities.py:1743)
@@ -221,7 +245,7 @@ def main():
         rec['edge_attr/%d' % i] = ea_list[i].numpy()
     for k, v in _np_state(model).items():
         rec['w/%s' % k] = v
-    np.savez_compressed(os.path.join(OUT, 'g5_mgkn_burgers1d.npz'), **rec)
+    _save('g5_mgkn_burgers1d.npz', **rec)
 
     # ---------------- G6: graph-generator restatement pins (edge lists from sklearn path) ----------
     rec = {}
@@ -231,7 +255,7 @@ def main():
         th = np.arange(s * s, dtype=np.float64) * 0.01
         rec['ei/%d_%g' % (s, r)] = ei.numpy().astype(np.int32)
         rec['ea/%d_%g' % (s, r)] = mg.attributes(theta=th).numpy()
-    np.savez_compressed(os.path.join(OUT, 'g6_ball_graphs.npz'), **rec)
+    _save('g6_ball_graphs.npz', **rec)
     # ---------------- G7: multi-level (MGKN) graph generator pins, RandomMultiMeshGenerator, seeded ----------
     s, m, ri, rx = 31, [200, 80, 30], [0.155, 0.31, 0.62], [0.21, 0.41]    # radii without lattice ties
     torch.manual_seed(0)
@@ -241,7 +265,7 @@ def main():
     r_mid, r_down, r_up = mmg.get_edge_index_range()
     theta = np.random.RandomState(0).randn(s * s)
     a_mid, a_down, a_up = mmg.attributes(theta=theta)
-    np.savez_compressed(os.path.join(OUT, 'g7_multilevel_graph.npz'), s=s, m=np.array(m), ri=np.array(ri),
+    _save('g7_multilevel_graph.npz', s=s, m=np.array(m), ri=np.array(ri),
                         rx=np.array(rx), theta=theta, e_mid=e_mid.numpy().astype(np.int32),
                         e_down=e_down.numpy().astype(np.int32), e_up=e_up.numpy().astype(np.int32),
                         r_mid=r_mid.numpy(), r_down=r_down.numpy(), r_up=r_up.numpy(),

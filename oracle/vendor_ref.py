@@ -1,17 +1,18 @@
-"""Put an UNMODIFIED copy of the reference's hot-path files under baseline/_ref/ (git-ignored, travels to the
-GPU box with the gpurun snapshot) so that `bench.py --impl reference` times the reference's OWN code.
+"""Put an UNMODIFIED copy of the reference's hot-path files under oracle/_ref/ (git-ignored build output) so that
+`bench.py --impl reference` times the reference's OWN code.
 
 TEST / MEASUREMENT INFRASTRUCTURE, never imported by the product path.
 
-The reference is a directory of scripts without setup.py / pyproject.toml, so
-`pip install --target baseline/_ref /root/reference` has nothing to install; this recipe is the equivalent:
-it copies, byte for byte,
+The reference is a directory of scripts without setup.py / pyproject.toml, so there is nothing to pip-install;
+this recipe is the equivalent: from the reference checkout (REF: $GRAPH_PDE_REFERENCE, default /root/reference) it
+copies, byte for byte,
     graph-neural-operator/nn_conv.py          (NNConv_old: the operator)
     graph-neural-operator/utilities.py        (DenseNet: the edge MLP)
     multipole-graph-neural-operator/utilities.py
-and records their sha256 in baseline/_ref/MANIFEST.json.  Third-party torch_geometric / torch_scatter are
-not installable here (no wheels, no network): the copied files run over oracle/pyg_stub, the restated
-MessagePassing boundary (see its docstring).  Nothing is copied into tracked paths.
+and records their sha256 in oracle/_ref/MANIFEST.json.  Third-party torch_geometric / torch_scatter are
+not needed: the copied files run over oracle/pyg_stub, the restated MessagePassing boundary (see its docstring).
+When REF is absent or unreadable nothing is copied and the benchmark's CPU baseline uses the oracle port instead.
+Nothing is copied into tracked paths.
 """
 import hashlib
 import json
@@ -20,9 +21,8 @@ import shutil
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(HERE)
-REF = '/root/reference'
-DST = os.path.join(ROOT, 'baseline', '_ref')
+DST = os.path.join(HERE, '_ref')
+REF = os.environ.get('GRAPH_PDE_REFERENCE') or '/root/reference'
 FILES = [
     ('graph-neural-operator/nn_conv.py', 'graph-neural-operator/nn_conv.py'),
     ('graph-neural-operator/utilities.py', 'graph-neural-operator/utilities.py'),
@@ -31,9 +31,9 @@ FILES = [
 
 
 def vendor(verbose=False):
-    """Returns True when baseline/_ref holds the files (copied now or earlier), False when there is no
+    """Returns True when oracle/_ref holds the files (copied now or earlier), False when there is no
     reference to copy from and nothing was vendored before."""
-    if not os.path.isdir(REF):
+    if not all(os.access(os.path.join(REF, src), os.R_OK) for src, _ in FILES):
         return os.path.exists(os.path.join(DST, 'MANIFEST.json'))
     manifest = {}
     for src, dst in FILES:

@@ -37,6 +37,26 @@ def cfg1_weights(g):
     return fc1, [l.weight.detach() for l in lins], [l.bias.detach() for l in lins], root, bias
 
 
+def vcycle_weights(g, variant):
+    """Parameters of the golden G4 model `variant` ('neurips1': KernelInduced, 'general': MKGN) as numpy arrays.
+    G4 stores their seed, shapes and sha256 instead of the values: they are re-drawn here with this project's
+    constructors, which draw the reference classes' init stream, and must hash to the reference's bytes."""
+    import hashlib
+    from graph_pde_b200.models import MKGN, KernelInduced
+    pts = [int(p) for p in g['points']]
+    cls = KernelInduced if variant == 'neurips1' else MKGN
+    with torch.random.fork_rng(devices=[]):
+        torch.manual_seed(int(g[variant + '/seed']))
+        model = cls(width=int(g['width']), ker_width=int(g['ker_width']), depth=int(g['depth']), ker_in=6, points=pts,
+                    level=len(pts), in_width=6)
+    st = {k: v.detach().numpy().copy() for k, v in model.state_dict().items()}
+    pre = variant + '/sha256/'
+    assert sorted(st) == sorted(k[len(pre):] for k in g.files if k.startswith(pre))
+    for k, v in st.items():
+        assert hashlib.sha256(v.tobytes()).hexdigest() == str(g[pre + k]), 're-drawn %s/%s differs' % (variant, k)
+    return st
+
+
 class DenseNetLike(torch.nn.Module):
     """Same module tree / state-dict keys as the reference's DenseNet (utilities.py:201-227):
     self.layers = ModuleList([Linear, ReLU, Linear, ..., Linear])."""

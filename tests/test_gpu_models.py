@@ -8,7 +8,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from tests.helpers import GOLDEN, TOL, cfg1_weights, ei64, rel_err, t
+from tests.helpers import GOLDEN, TOL, cfg1_weights, ei64, rel_err, t, vcycle_weights
 
 pytestmark = [pytest.mark.gpu, pytest.mark.usefixtures('edge_kernel_mode')]
 DEV = 'cuda:0'
@@ -60,8 +60,7 @@ def test_mgkn_vcycle(variant, precision, steps, monkeypatch):
     cls = KernelInduced if variant == 'neurips1' else MKGN
     model = cls(width=32, ker_width=64, depth=2, ker_in=6, points=pts, level=len(pts), in_width=6,
                 precision=precision)
-    pre = variant + '/w/'
-    model = _load(model, {k[len(pre):]: g[k] for k in g.files if k.startswith(pre)})
+    model = _load(model, vcycle_weights(g, variant))
     d = _Data()
     d.x = t(g['node_x']).to(DEV)
     for nm in ('mid', 'down', 'up'):
@@ -116,7 +115,7 @@ def test_cuda_graph_replay_of_kernelnn_and_vcycle():
     g4 = np.load(os.path.join(GOLDEN, 'g4_mgkn_vcycle.npz'))
     pts = [int(p) for p in g4['points']]
     vm = KernelInduced(width=32, ker_width=64, depth=2, ker_in=6, points=pts, level=len(pts), in_width=6)
-    vm = _load(vm, {k[len('neurips1/w/'):]: g4[k] for k in g4.files if k.startswith('neurips1/w/')})
+    vm = _load(vm, vcycle_weights(g4, 'neurips1'))
     dv = _Data()
     dv.x = t(g4['node_x']).to(DEV)
     for nm in ('mid', 'down', 'up'):

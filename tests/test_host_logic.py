@@ -11,7 +11,7 @@ from graph_pde_b200 import graphs
 from graph_pde_b200.models import DenseNet, KernelInduced, KernelNN, MGKN, MKGN
 from graph_pde_b200.nn_conv import NNConv, NNConv_old, _linear_chain
 from oracle import nnconv_oracle as O
-from tests.helpers import GOLDEN
+from tests.helpers import GOLDEN, vcycle_weights
 
 
 def test_signature_attributes_repr_and_state_dict_keys():
@@ -54,7 +54,7 @@ def test_whole_module_pickle_roundtrip(tmp_path):
 def test_checkpoint_state_dict_loads_into_our_kernelnn():
     g = np.load(os.path.join(GOLDEN, 'g3_checkpoint_grain_new.npz'))
     st = {k[2:]: torch.from_numpy(g[k]) for k in g.files if k.startswith('w/')}
-    mlp = DenseNet([6, 64, 128, 4096], torch.nn.ReLU)
+    mlp = DenseNet([6, 64, 32, 4096], torch.nn.ReLU)
     conv = NNConv_old(64, 64, mlp, aggr='mean')
     conv.load_state_dict({k[len('conv1.'):]: v for k, v in st.items() if k.startswith('conv1.')})
     assert torch.equal(conv.nn.layers[4].weight.detach(), st['conv1.nn.layers.4.weight'])
@@ -81,13 +81,15 @@ def test_model_constructors_match_reference_layouts():
     g = np.load(os.path.join(GOLDEN, 'g4_mgkn_vcycle.npz'))
     pts = [int(p) for p in g['points']]
     ki = KernelInduced(width=32, ker_width=64, depth=2, ker_in=6, points=pts, level=len(pts), in_width=6)
-    ref_keys = sorted(k[len('neurips1/w/'):] for k in g.files if k.startswith('neurips1/w/'))
+    ref_keys = sorted(k[len('neurips1/shape/'):] for k in g.files if k.startswith('neurips1/shape/'))
     assert sorted(ki.state_dict().keys()) == ref_keys
     for k in ref_keys:
-        assert tuple(ki.state_dict()[k].shape) == g['neurips1/w/' + k].shape, k
+        assert tuple(ki.state_dict()[k].shape) == tuple(g['neurips1/shape/' + k]), k
     mk = MKGN(width=32, ker_width=64, depth=2, ker_in=6, points=pts, level=len(pts), in_width=6)
-    ref_keys = sorted(k[len('general/w/'):] for k in g.files if k.startswith('general/w/'))
+    ref_keys = sorted(k[len('general/shape/'):] for k in g.files if k.startswith('general/shape/'))
     assert sorted(mk.state_dict().keys()) == ref_keys
+    for k in ref_keys:
+        assert tuple(mk.state_dict()[k].shape) == tuple(g['general/shape/' + k]), k
     g5 = np.load(os.path.join(GOLDEN, 'g5_mgkn_burgers1d.npz'))
     mg = MGKN(width=32, ker_width=64, depth=2, ker_in=4, in_width=2, s=int(g5['s']))
     ref_keys = sorted(k[2:] for k in g5.files if k.startswith('w/'))
@@ -220,8 +222,7 @@ def test_vcycle_step_chain_on_preactivations_equals_the_reference_op_sequence(mo
     g = np.load(os.path.join(GOLDEN, 'g4_mgkn_vcycle.npz'))
     pts = [int(p) for p in g['points']]
     model = models.KernelInduced(width=32, ker_width=64, depth=2, ker_in=6, points=pts, level=len(pts), in_width=6)
-    pre = 'neurips1/w/'
-    model.load_state_dict({k[len(pre):]: torch.from_numpy(g[k]) for k in g.files if k.startswith(pre)})
+    model.load_state_dict({k: torch.from_numpy(v) for k, v in vcycle_weights(g, 'neurips1').items()})
 
     class D(object):
         pass

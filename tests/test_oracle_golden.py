@@ -6,6 +6,7 @@ import numpy as np
 import torch
 
 from oracle import nnconv_oracle as O
+from tests.helpers import vcycle_weights
 
 TOL = dict(rtol=2e-5, atol=2e-5)     # fp32 vs fp32, summation order differs only by chunking
 
@@ -73,7 +74,7 @@ def test_g3_checkpoint_weights_stack(golden_dir):
     g = np.load(os.path.join(golden_dir, 'g3_checkpoint_grain_new.npz'))
     st = {k[2:]: _t(g[k]) for k in g.files if k.startswith('w/')}
     ws, bs = O.mlp_params_from_state(st, 'conv1.nn.')
-    assert [tuple(w.shape) for w in ws] == [(64, 6), (128, 64), (4096, 128)]
+    assert [tuple(w.shape) for w in ws] == [(64, 6), (32, 64), (4096, 32)]
     ei, ea = _ei(g['edge_index']), _t(g['edge_attr'])
     x = _t(g['x0'])
     out = O.kernelnn_conv_stack(x, ei, ea, ws, bs, st['conv1.root'], st['conv1.bias'], 6)
@@ -90,7 +91,7 @@ def test_g4_mgkn_vcycle_both_variants(golden_dir):
                 range_mid=g['range_mid'], range_down=g['range_down'], range_up=g['range_up'])
     pts = [int(p) for p in g['points']]
     for variant in ('neurips1', 'general'):
-        st = {k[len(variant) + 3:]: _t(g[k]) for k in g.files if k.startswith(variant + '/w/')}
+        st = {k: _t(v) for k, v in vcycle_weights(g, variant).items()}
         out = O.mgkn_vcycle_forward(_t(g['node_x']), data, st, int(g['depth']), len(pts), pts, variant)
         np.testing.assert_allclose(out.numpy(), g[variant + '/out'], rtol=1e-4, atol=1e-5)
 
